@@ -2,7 +2,7 @@
 """bench.py — benchmark of the per-block audio-graph DSP path (BASELINE.json metric: mono-equivalent samples/s through
 the graph at 1/2/4/8 B200; conv-reverb TFLOPS).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--only c2,c3,c4,c5,dag]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--only c2,c3,c4,c5,dag] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic input. ONE JSON line on rank 0:
   headline (`value`, `ms_per_step`, `roofline`, `e2e`, `cpu_baseline`) = c2, BASELINE configs[1]: 1024 stereo voices per GPU,
@@ -15,9 +15,12 @@ A *step* is one pass of the hot path over one batch of synthetic input. ONE JSON
       dag a non-chain voice graph (dry + SVF send + biquad send -> 6-port SumNode -> pan -> bus) on the generic lowering, plus block-sized
           calls (one 256-frame block per call) replayed from a captured CUDA graph: us per call;
   `cpu_baseline.c1` = configs[0]: one VolumeNode, mono, 256-frame blocks on the CPU oracle (ns per block of executor plumbing).
-Timing: every config is timed over >= ~1 s as R passes of exactly `--steps` steps; a pass is bracketed by a barrier and a
-stream synchronise on both sides and timed with CUDA events on the processor's stream; per pass the MAX over ranks is
-taken, then the median over passes (p10 / p90 reported).
+Timing: every config runs max(W, 3) untimed warm-up steps, then exactly `--steps` timed steps back to back, bracketed by a
+barrier and a stream synchronise on both sides and timed with CUDA events on the processor's stream; the MAX over ranks is
+taken. The step count before the last timed step is fixed by the arguments, so stateful configs end in the same state.
+`--dump-outputs DIR` writes, per config, the output of the last timed step (what the caller of the timed path receives: the
+master bus, or the per-voice outputs) as DIR/<config>.npy (float32, rank 0's); a config whose output exceeds its share of
+64 MB keeps a fixed, seeded sample of whole voices (rows of axis 0, in ascending order).
 N > 1 is launched by torchrun (one rank per GPU) but uses no torch: the communicator id travels through a file, barriers
 and reductions through the product's own NCCL communicator (firewheel_b200/rendezvous.py).
 `--impl reference` times the CPU oracle (the C++ restatement of the reference's Rust path — Rust cannot be built in
@@ -26,7 +29,6 @@ this image) on all host cores over the headline workload.
 import argparse
 import ctypes
 import json
-import math
 import os
 import statistics
 import subprocess
@@ -68,6 +70,7 @@ WORKLOADS["dag"] = dict(voices=1024, ch=2, block=256, blocks=64, bus=True, bytes
                         kernel="generic lowering: chain_kernel (gain / pan / copies), biquad_delay_lanes (SVF, biquad), sum_kernel, bus tree",
                         desc="dag: 1024 stereo voices/GPU, graph_in -> {gain | 2-stage SVF -> gain | 2-stage biquad -> gain} -> 6-port SumNode -> pan -> master bus, 256-frame blocks, 64 blocks/step")
 REVERB_WORKLOADS = ("c4", "c5")
+DUMP_LIMIT_BYTES = 64_000_000  # all --dump-outputs files of one run together
 
 
 def synth(shape, seed):
@@ -390,11 +393,17 @@ class Comm:
     def max(self, a):
         return self.gather(np.asarray(a, np.float64)).max(axis=0)
 
-    def bcast0(self, a):
-        return self.gather(np.asarray(a))[0]
+
+def dump_output(out_dir, name, y, limit):
+    """`y` as out_dir/<name>.npy; above `limit` bytes, a seeded sample of its rows (voices) in ascending order."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    if y.nbytes > limit:
+        n = max(1, limit // (y.nbytes // y.shape[0]))
+        y = y[np.sort(np.random.default_rng(0).choice(y.shape[0], n, replace=False))]
+    np.save(out_dir / f"{name}.npy", np.ascontiguousarray(y, F32))
 
 
-def run_config(fw, lib, name, args, rank, world, local_rank, want_cpu):
+def run_config(fw, lib, name, args, rank, world, local_rank, want_cpu, dump_bytes):
     from firewheel_b200 import rendezvous
     w = WORKLOADS[name]
     C, F, KB = w["ch"], w["block"], w["blocks"]
@@ -448,24 +457,24 @@ def run_config(fw, lib, name, args, rank, world, local_rank, want_cpu):
 
     for _ in range(max(args.warmup, 3)):
         step()
-    est = float(comm.max([one_pass(args.steps)])[0])
-    n_pass = int(min(2000, max(5, math.ceil(args.min_seconds * 1e3 / max(est, 1e-3)))))
-    n_pass = int(comm.bcast0(np.array([n_pass], np.int64))[0])
     clocks = ClockSampler(local_rank)
     clocks.start()
     launches0 = proc.kernel_launches()
-    mine = np.array([one_pass(args.steps) for _ in range(n_pass)], np.float64)
-    launches = (proc.kernel_launches() - launches0) // n_pass
+    mine = one_pass(args.steps)
+    launches = proc.kernel_launches() - launches0
     clk = clocks.stop()
-    per_pass = comm.max(mine)  # max over ranks, pass by pass
-    by_rank = [float(v) / args.steps for v in comm.gather(np.array([np.median(mine)], np.float64))[:, 0]]  # each rank's own median: GPUs of one box differ
-    ms_per_step = float(np.median(per_pass)) / args.steps
-    p10, p90 = (float(np.percentile(per_pass, q)) / args.steps for q in (10, 90))
+    if dump_bytes and rank == 0:
+        proc.d2h(h_out, d_out, out_bytes)
+        proc.sync()
+        dump_output(Path(args.dump_outputs), name, y, dump_bytes)
+    timed_ms = float(comm.max([mine])[0])
+    by_rank = [float(v) / args.steps for v in comm.gather(np.array([mine], np.float64))[:, 0]]  # GPUs of one box differ
+    ms_per_step = timed_ms / args.steps
     samples_per_step = V * C * T * world
     value = samples_per_step / (ms_per_step * 1e-3)
 
     # per-kernel-class pass: a CUDA-event pair around every kernel class (these events serialise the programmatic-dependent-
-    # launch overlap, so they stay out of the timed passes)
+    # launch overlap, so they stay out of the timed window)
     proc.profile(True)
     prof_steps = max(args.steps, 5)
     for _ in range(prof_steps):
@@ -551,12 +560,12 @@ def run_config(fw, lib, name, args, rank, world, local_rank, want_cpu):
                       "note": "256-frame block for 1024 voices per call through fw_processor_process_planar_device; realtime budget of one block at 48 kHz is 5333 us"}
 
     res = {"metric": "mono_equiv_samples_per_sec", "value": value, "unit": "samples/s", "ms_per_step": ms_per_step,
-           "ms_per_step_p10": p10, "ms_per_step_p90": p90, "ms_per_step_by_rank": by_rank, "passes": n_pass, "steps_per_pass": args.steps, "timed_seconds": float(per_pass.sum()) * 1e-3,
+           "ms_per_step_by_rank": by_rank, "timed_steps": args.steps, "timed_seconds": timed_ms * 1e-3,
            "scaling": w["scaling"], "dtype": "bf16 x bf16 -> f32 (FIR), f32 elsewhere" if tensor else "f32",
            "config": cfg_dict(name, V, world), "clocks": clk,
            "e2e": {"value": samples_per_step / e2e_s, "unit": "samples/s", "h2d_bytes_per_step": in_bytes * world, "d2h_bytes_per_step": out_bytes * world,
                    "steps": e2e_steps, "ms_per_step": e2e_s * 1e3, "api": "fw_processor_process_planar (pinned host buffers)"},
-           "gpu_launches_per_pass": int(launches), "roofline": roofline, "parity": parity, "cpu_baseline": cpu}
+           "gpu_launches_timed": int(launches), "roofline": roofline, "parity": parity, "cpu_baseline": cpu}
     if block_call:
         res["block_sized_calls"] = block_call
     if tensor:
@@ -647,10 +656,11 @@ def run_b200(args, rank, world, local_rank):
             os.environ["NCCL_DEBUG"] = "NONE"
     names = [n for n in args.only.split(",") if n]
     want_cpu = world == 1 and not os.environ.get("FW_BENCH_SKIP_CPU")
+    dump_bytes = DUMP_LIMIT_BYTES // len(names) - 4096 if args.dump_outputs else 0  # 4096: room for the .npy header
     results = {}
     for n in names:
         t0 = time.perf_counter()
-        results[n] = run_config(fw, lib, n, args, rank, world, local_rank, want_cpu)
+        results[n] = run_config(fw, lib, n, args, rank, world, local_rank, want_cpu, dump_bytes)
         results[n]["bench_wall_s"] = time.perf_counter() - t0
     rendezvous.cleanup(rank)
     if rank != 0:
@@ -660,8 +670,8 @@ def run_b200(args, rank, world, local_rank):
     line = {"metric": "mono_equiv_samples_per_sec", "value": head["value"], "unit": "samples/s", "n_gpus": world, "steps": args.steps,
             "warmup": max(args.warmup, 3), "ms_per_step": head["ms_per_step"], "higher_is_better": True, "scaling": head["scaling"], "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": head["config"], "clocks": head["clocks"], "e2e": head["e2e"],
-            "gpu_launches": head["gpu_launches_per_pass"], "roofline": head["roofline"], "cpu_baseline": head["cpu_baseline"]}
-    for k in ("ms_per_step_p10", "ms_per_step_p90", "ms_per_step_by_rank", "passes", "timed_seconds", "parity", "exchange", "bus_parity", "bus_identical_on_all_ranks", "block_sized_calls"):
+            "gpu_launches": head["gpu_launches_timed"], "roofline": head["roofline"], "cpu_baseline": head["cpu_baseline"]}
+    for k in ("ms_per_step_by_rank", "timed_seconds", "parity", "exchange", "bus_parity", "bus_identical_on_all_ranks", "block_sized_calls"):
         if k in head:
             line[k] = head[k]
     if want_cpu and line["cpu_baseline"] is not None:
@@ -678,10 +688,15 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--only", default="c2,c3,c4,c5,dag", help="comma-separated configs to run (the first of c2 / the list is the headline)")
     ap.add_argument("--workload", default=None, help="alias of --only for a single config")
-    ap.add_argument("--min-seconds", type=float, default=1.0, dest="min_seconds", help="timed seconds per config")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", dest="dump_outputs",
+                    help="write each config's output of the last timed step to DIR/<config>.npy (at most 64 MB in all)")
     args = ap.parse_args()
     if args.workload:
         args.only = args.workload
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
